@@ -67,7 +67,34 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-mode", action="store_true",
                     help="warm-up + device-resident loop only (for ncu launch lists); prints no bench line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64; 64 MB in all, "
+                         "a seeded sample of rows where an output is larger than its share), to compare two builds")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl r3g: the reference arm times bounded samples and keeps no outputs")
+    return args
+
+
+DUMP_BYTES = 60 << 20      # the arrays' data: with the .npy headers the files stay under 64 MB (64e6 bytes)
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: every array as <path>/<name>.npy, float32 kept and any other dtype as float64.  The arrays share
+    DUMP_BYTES equally; one larger than its share is viewed as rows of its last dimension and replaced by a fixed,
+    seeded sample of those rows in their original order, so two builds that compute the same outputs write the same
+    files."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if a.nbytes > share:
+            rows = a.reshape(-1, a.shape[-1])
+            keep = share // rows[0].nbytes
+            a = rows[np.sort(np.random.default_rng(0).choice(len(rows), keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def peaks():
@@ -359,6 +386,7 @@ def main_shapegen(args):
     launches0 = ctx.launches + pipe.replayed_launches
     h2d = 0
     meshes = []
+    kept = {}                          # --dump-outputs: the meshes of the last timed step
     seg_dev, seg_e2e = [], []
 
     def mark():
@@ -374,6 +402,8 @@ def main_shapegen(args):
         seg_dev.append((a, mark()))
         if k == 0:      # only the first mesh is kept (for the line's statistics): holding all K would make every later
             meshes.append(m)    # object cudaMalloc fresh ~200 MB blocks (100 ms each) inside the timed region
+        if args.dump_outputs and k == K - 1:
+            kept["resident"] = m
 
     host = {"pipe_call_ms": 0.0, "gather_submit_ms": 0.0}      # host wall time of the two halves of an e2e step
 
@@ -388,6 +418,8 @@ def main_shapegen(args):
         host["pipe_call_ms"] += 1e3 * (t1 - t0) / K
         host["gather_submit_ms"] += 1e3 * (time.perf_counter() - t1) / K
         seg_e2e.append((a, mark()))
+        if args.dump_outputs and k == K - 1:
+            kept["e2e"] = m2
 
     barrier()
     if args.profile_mode:
@@ -427,6 +459,10 @@ def main_shapegen(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_dev, ms_e2e = t.tolist()
     stage = dict(pipe.timings)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f"{arm}_mesh_{part}": getattr(m, attr)
+                                         for arm, m in kept.items() if m is not None
+                                         for part, attr in (("vertices", "mesh_v"), ("faces", "mesh_f"))})
     if args.profile_mode:
         if rank == 0:
             print(json.dumps({"profile_mode": True, "ms_per_step": ms_dev / K, "stages_ms_last_object": stage}))
@@ -523,8 +559,12 @@ def main_vggt(args):
     h2d = d2h = 0
     barrier()
     ev[0].record()
+    kept = {}                          # --dump-outputs: what the last timed step's device-resident scene returned
     for k in range(K):
-        scene(dev_in[W + k])
+        res = scene(dev_in[W + k])
+        if args.dump_outputs and k == K - 1:
+            kept = dict(zip(("resident_points", "resident_depth", "resident_conf"), res))
+        del res
         ev[2 * k + 1].record()
         img = host_in[W + k].cuda(non_blocking=True)
         h2d += host_in[W + k].numel() * 4
@@ -543,6 +583,8 @@ def main_vggt(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_dev, ms_e2e = t.tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(kept, e2e_points=host_pts, e2e_depth=host_dc[0], e2e_conf=host_dc[1]))
     if rank == 0:
         # roofline: the back-projection kernel on a shape long enough to read a bandwidth (SURVEY.md section 8d row 4:
         # the real 2 x 518^2 call is 8.6 MB = launch-latency bound)

@@ -7,6 +7,9 @@ Run in the build container only:  python oracle/make_golden.py
 The reference ships no weights and no golden vectors of its own (SURVEY.md section 4), so these
 fixtures are the pin: weights are the modules' default initialisation under torch.manual_seed,
 rounded through fp16 (what a GPU run holds) and evaluated in fp32 on the CPU.
+Where the weights or an output are too large to store, a fixture keeps the state-dict layout (filled by
+seeded_weights) or a digest of the output's bytes; the tests import those helpers and the seeded test
+inputs from here, so they run without the reference.
 """
 import os
 import sys
@@ -32,6 +35,64 @@ def fp16_round_(module, buffers=True):
 
 def sd_np(module, prefix=""):
     return {"w:" + prefix + k: v.detach().half().numpy() for k, v in module.state_dict().items()}
+
+
+def layout_np(module, prefix=""):
+    """The state-dict layout of a module (key -> shape) as "shape:<prefix><key>" entries of a fixture."""
+    return {"shape:" + prefix + k: np.array(v.shape, np.int64) for k, v in module.state_dict().items()}
+
+
+def stored_layout(z, prefix=""):
+    """{key: shape} of the "shape:<prefix>..." entries of a fixture (or of a dict) written with layout_np."""
+    return {k[len("shape:"):]: tuple(int(s) for s in z[k]) for k in z if k.startswith("shape:" + prefix)}
+
+
+def seeded_weights(shapes, seed=0):
+    """float32 tensors for a {key: shape} layout, drawn in sorted key order from one seeded stream, so that a fixture
+    only needs to store the layout: matrices and kernels U(-1, 1) / sqrt(fan_in), 1-d norm scales (`*weight`,
+    `*scale`) 1 + 0.2 N(0, 1), everything else (biases, LayerScale gammas, tokens) 0.2 N(0, 1)."""
+    rng = np.random.default_rng(seed)
+    out = {}
+    for k in sorted(shapes):
+        shape = tuple(shapes[k])
+        if len(shape) >= 2:
+            v = rng.uniform(-1.0, 1.0, shape) / np.sqrt(np.prod(shape[1:]))
+        elif k.endswith(("weight", "scale")):
+            v = 1.0 + 0.2 * rng.standard_normal(shape)
+        else:
+            v = 0.2 * rng.standard_normal(shape)
+        out[k] = torch.from_numpy(v.astype(np.float32))
+    return out
+
+
+def sha256(t):
+    """Digest of a tensor's or array's bytes: pins a large output that must match bit for bit."""
+    import hashlib
+    a = t.numpy() if isinstance(t, torch.Tensor) else t
+    return np.str_(hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest())
+
+
+def ellipse_rgba():
+    """300x420 RGBA: seeded noise RGB inside an elliptical alpha mask (the image processor's test input)."""
+    rng = np.random.default_rng(0)
+    rgba = np.zeros((300, 420, 4), np.uint8)
+    rgba[..., :3] = rng.integers(0, 256, (300, 420, 3))
+    yy, xx = np.mgrid[0:300, 0:420]
+    rgba[..., 3] = ((((xx - 200) / 120) ** 2 + ((yy - 160) / 90) ** 2) <= 1) * 255
+    return rgba
+
+
+def loader_pngs(directory):
+    """Three seeded PNGs (landscape RGB, portrait RGBA, square RGB) for the square image loader."""
+    from PIL import Image
+    rng = np.random.default_rng(9)
+    paths = []
+    for i, (w, h, mode) in enumerate(((150, 100, "RGB"), (64, 97, "RGBA"), (80, 80, "RGB"))):
+        arr = rng.integers(0, 256, (h, w, 4 if mode == "RGBA" else 3)).astype(np.uint8)
+        path = os.path.join(str(directory), f"im{i}.png")
+        Image.fromarray(arr, mode).save(path)
+        paths.append(path)
+    return paths
 
 
 def golden_dit():
@@ -266,6 +327,107 @@ def golden_vggt():
     print("vggt_mini: outs", len(outs), tuple(outs[0].shape))
 
 
+def golden_checkpoint_layout():
+    """State-dict layout of a `model.fp16.safetensors` (pipelines.py:140-232) at the small sizes of
+    tests/test_checkpoint_loading.py: the reference's Hunyuan3DDiT ("model."), ShapeVAE transformer and geo-decoder
+    ("vae.").  The test fills it with seeded_weights."""
+    m = ref_import.hunyuan_dit()
+    ab, _, _ = ref_import.hunyuan_autoencoders()
+    dit = m.Hunyuan3DDiT(in_channels=64, context_in_dim=96, hidden_size=128, mlp_ratio=4.0, num_heads=2, depth=2,
+                         depth_single_blocks=3, axes_dim=[64], theta=10000, qkv_bias=True, time_factor=1000,
+                         guidance_embed=False)
+    tr = ab.Transformer(n_ctx=48, width=128, layers=2, heads=2, qkv_bias=False, qk_norm=True)
+    geo = ab.CrossAttentionDecoder(out_channels=1, num_latents=48, mlp_expand_ratio=4, downsample_ratio=1,
+                                   enable_ln_post=True, fourier_embedder=ab.FourierEmbedder(num_freqs=8, include_pi=False),
+                                   width=128, heads=2, qkv_bias=False, qk_norm=True, label_type="binary")
+    d = layout_np(dit, "model.")
+    d.update(layout_np(torch.nn.Linear(64, 128), "vae.post_kl."))
+    d.update(layout_np(tr, "vae.transformer."))
+    d.update(layout_np(geo, "vae.geo_decoder."))
+    np.savez_compressed(os.path.join(OUT, "checkpoint_layout.npz"), **d)
+    print("checkpoint_layout:", len(d), "tensors")
+
+
+def golden_vggt_heads():
+    """CameraHead / DPTHead (vggt/heads/camera_head.py, dpt_head.py) and pose_encoding_to_extri_intri (pose_enc.py) in
+    fp32 on the CPU: seeded_weights of the heads' layout, tokens and images from torch.manual_seed(0)."""
+    ref_import.vggt_package()
+    from vggt.heads.camera_head import CameraHead
+    from vggt.heads.dpt_head import DPTHead
+    from vggt.utils.pose_enc import pose_encoding_to_extri_intri
+    C, S, H, W = 128, 2, 56, 70
+    torch.manual_seed(0)
+    toks = [torch.randn(1, S, 5 + (H // 14) * (W // 14), C) for _ in range(4)]
+    imgs = torch.rand(1, S, 3, H, W)
+    cam = CameraHead(dim_in=C, trunk_depth=2, num_heads=2).eval()
+    dpt = DPTHead(dim_in=C, output_dim=2, activation="exp", conf_activation="expp1", features=32,
+                  out_channels=[16, 32, 64, 64], intermediate_layer_idx=[0, 1, 2, 3]).eval()
+    d = layout_np(cam, "camera_head.")
+    d.update(layout_np(dpt, "depth_head."))
+    w = seeded_weights(stored_layout(d))
+    for prefix, mod in (("camera_head.", cam), ("depth_head.", dpt)):
+        mod.load_state_dict({k[len(prefix):]: v for k, v in w.items() if k.startswith(prefix)})
+    with torch.no_grad():
+        poses = cam(toks)
+        depth, conf = dpt(toks, images=imgs, patch_start_idx=5)
+    extrinsic, intrinsic = pose_encoding_to_extri_intri(poses[-1], (H, W))
+    for i, p in enumerate(poses):
+        d[f"pose{i}"] = p.numpy()
+    d.update(extrinsic=extrinsic.numpy(), intrinsic=intrinsic.numpy(), depth=depth.numpy(), conf=conf.numpy())
+    np.savez_compressed(os.path.join(OUT, "vggt_heads_mini.npz"), **d)
+    print("vggt_heads_mini: depth", tuple(depth.shape), "range", float(depth.min()), float(depth.max()))
+
+
+def golden_host_helpers():
+    """Host-side helpers of the pipeline and the stage scripts, on the inputs of tests/test_host_logic.py and
+    tests/test_stage4_tail.py: ImageProcessorV2 (preprocessors.py), DinoImageEncoder (conditioner.py:57-131) with
+    seeded_weights, extract_near_surface_volume_fn (volume_decoders.py:29-119), vggt/utils/helper.py and
+    load_and_preprocess_images_square (vggt/utils/load_fn.py:13-94).  The two image outputs that must match bit for
+    bit are stored as digests of their bytes."""
+    import tempfile
+    import warnings
+    from PIL import Image
+    d = {}
+    out = ref_import.hunyuan_preprocessors().ImageProcessorV2(size=512, border_ratio=0.15)(
+        Image.fromarray(ellipse_rgba(), "RGBA"))
+    d["imgproc_image_sha256"], d["imgproc_mask_sha256"] = sha256(out["image"]), sha256(out["mask"])
+
+    cfg = dict(hidden_size=32, num_hidden_layers=2, num_attention_heads=2, mlp_ratio=2, patch_size=14, image_size=56,
+               use_swiglu_ffn=True, layerscale_value=1.0, qkv_bias=True, hidden_act="gelu", layer_norm_eps=1e-6)
+    enc = ref_import.hunyuan_conditioner().DinoImageEncoder(config=cfg, use_cls_token=True, image_size=56)
+    enc.model.load_state_dict(seeded_weights({k: v.shape for k, v in enc.model.state_dict().items()}))
+    g = torch.Generator().manual_seed(0)
+    with torch.no_grad():
+        for i, shape in enumerate(((1, 3, 70, 90), (2, 3, 100, 64), (1, 3, 56, 56))):
+            d[f"dino_out{i}"] = enc(torch.rand(shape, generator=g) * 2 - 1).numpy()
+    d["dino_uncond"] = enc.unconditional_embedding(2).numpy()
+
+    _, _, vd = ref_import.hunyuan_autoencoders()
+    torch.manual_seed(0)
+    for n in (5, 9):
+        x = torch.randn(n, n, n)
+        x[torch.rand(n, n, n) < 0.25] = -10000.0
+        for j, alpha in enumerate((0.0, 0.3, -0.2)):
+            with warnings.catch_warnings():
+                warnings.simplefilter("ignore")
+                d[f"near_surface_{n}_{j}"] = vd.extract_near_surface_volume_fn(x.clone(), alpha).numpy()
+
+    ref_import.vggt_package()
+    from vggt.utils import helper
+    from vggt.utils.load_fn import load_and_preprocess_images_square
+    d["pixel_grid"] = helper.create_pixel_coordinate_grid(2, 5, 4)
+    np.random.seed(7)
+    d["limited_mask"] = helper.randomly_limit_trues(np.random.default_rng(3).random((2, 30, 30)) > 0.3, 100)
+    with tempfile.TemporaryDirectory() as tmp:
+        paths = loader_pngs(tmp)
+        for tag, sel in (("3", paths), ("1", paths[:1])):
+            img, xy = load_and_preprocess_images_square(sel, 256)
+            d[f"loader{tag}_sha256"], d[f"loader{tag}_shape"], d[f"loader{tag}_coords"] = (
+                sha256(img), np.array(img.shape, np.int64), xy.numpy())
+    np.savez_compressed(os.path.join(OUT, "host_helpers.npz"), **d)
+    print("host_helpers:", len(d), "arrays")
+
+
 if __name__ == "__main__":
     assert ref_import.available(), "reference checkout not found"
     os.makedirs(OUT, exist_ok=True)
@@ -276,3 +438,6 @@ if __name__ == "__main__":
     golden_scheduler()
     golden_unproject()
     golden_vggt()
+    golden_checkpoint_layout()
+    golden_vggt_heads()
+    golden_host_helpers()

@@ -63,6 +63,10 @@ def hunyuan_preprocessors():
     return _load_file("_ref_preprocessors", os.path.join(HY, "hy3dgen/shapegen/preprocessors.py"))
 
 
+def hunyuan_conditioner():
+    return _load_file("_ref_conditioner", os.path.join(HY, "hy3dgen/shapegen/models/conditioner.py"))
+
+
 def vggt_package():
     if VGGT not in sys.path:
         sys.path.insert(0, VGGT)

@@ -1,12 +1,13 @@
 """CPU: `Hunyuan3DDiTFlowMatchingPipeline.from_pretrained` on a fabricated checkpoint in the reference's layout
 ($HY3DGEN_MODELS/<repo>/<subfolder>/config.yaml + model.fp16.safetensors with `model.` / `vae.` / `conditioner.` key
-prefixes, pipelines.py:140-232).  The tensors come from modules built with the reference's own classes (small sizes), so
-the test pins the state-dict key mapping, the linear1 row permutation and the modulation packing -- the part of the
-drop-in that no GPU test can reach because no real checkpoint is reachable here."""
+prefixes, pipelines.py:140-232).  The DiT / VAE key names and shapes are the state-dict layout of the reference's own
+classes at small sizes (tests/golden/checkpoint_layout.npz, oracle/make_golden.py) filled with seeded values, so the
+test pins the state-dict key mapping, the linear1 row permutation and the modulation packing -- the part of the drop-in
+that no GPU test can reach because no real checkpoint is reachable here."""
 import os
 import sys
 
-import pytest
+import numpy as np
 import torch
 import yaml
 
@@ -15,14 +16,10 @@ sys.path.insert(0, os.path.join(ROOT, "3d-re-gen_b200"))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 
-def test_from_pretrained_maps_a_reference_layout_checkpoint(tmp_path, monkeypatch):
-    import ref_import
-    if not ref_import.available():
-        pytest.skip("/root/reference not present")
+def test_from_pretrained_maps_a_reference_layout_checkpoint(tmp_path, monkeypatch, golden_dir):
     import safetensors.torch
+    from make_golden import seeded_weights, stored_layout
     from transformers import Dinov2Config, Dinov2Model
-    ref_dit = ref_import.hunyuan_dit()
-    ab, _, _ = ref_import.hunyuan_autoencoders()
     H, Mh, nh = 128, 512, 2
     dit_p = dict(in_channels=64, context_in_dim=96, hidden_size=H, mlp_ratio=4.0, num_heads=nh, depth=2,
                  depth_single_blocks=3, axes_dim=[64], theta=10000, qkv_bias=True, time_factor=1000, guidance_embed=False)
@@ -30,20 +27,10 @@ def test_from_pretrained_maps_a_reference_layout_checkpoint(tmp_path, monkeypatc
                  qkv_bias=False, qk_norm=True, scale_factor=0.999)
     dino_p = dict(hidden_size=96, num_hidden_layers=2, num_attention_heads=2, mlp_ratio=2, patch_size=14, image_size=56,
                   use_swiglu_ffn=True, layerscale_value=1.0, qkv_bias=True, hidden_act="gelu", layer_norm_eps=1e-6)
+    layout = stored_layout(np.load(os.path.join(golden_dir, "checkpoint_layout.npz")))
+    flat = {k: v.half() for k, v in seeded_weights(layout).items()}
     torch.manual_seed(0)
-    dit = ref_dit.Hunyuan3DDiT(**dit_p)
-    post_kl = torch.nn.Linear(64, 128)
-    tr = ab.Transformer(n_ctx=48, width=128, layers=2, heads=2, qkv_bias=False, qk_norm=True)
-    geo = ab.CrossAttentionDecoder(out_channels=1, num_latents=48, mlp_expand_ratio=4, downsample_ratio=1,
-                                   enable_ln_post=True, fourier_embedder=ab.FourierEmbedder(num_freqs=8, include_pi=False),
-                                   width=128, heads=2, qkv_bias=False, qk_norm=True, label_type="binary")
     dino = Dinov2Model(Dinov2Config(**dino_p))
-    flat = {}
-    for k, v in dit.state_dict().items():
-        flat["model." + k] = v.half().contiguous()
-    for prefix, mod in (("vae.post_kl.", post_kl), ("vae.transformer.", tr), ("vae.geo_decoder.", geo)):
-        for k, v in mod.state_dict().items():
-            flat[prefix + k] = v.half().contiguous()
     for k, v in dino.state_dict().items():
         flat["conditioner.main_image_encoder.model." + k] = v.half().contiguous()
     base = tmp_path / "tencent" / "Hunyuan3D-2" / "hunyuan3d-dit-v2-0"
@@ -63,7 +50,7 @@ def test_from_pretrained_maps_a_reference_layout_checkpoint(tmp_path, monkeypatc
     monkeypatch.setenv("HY3DGEN_MODELS", str(tmp_path))
     from r3g.pipelines import Hunyuan3DDiTFlowMatchingPipeline
     pipe = Hunyuan3DDiTFlowMatchingPipeline.from_pretrained("tencent/Hunyuan3D-2", device="cpu")
-    w, sd = pipe.model.w, {k: v.half() for k, v in dit.state_dict().items()}
+    w, sd = pipe.model.w, {k[len("model."):]: v for k, v in flat.items() if k.startswith("model.")}
     # plain tensors keep their keys
     for k in ("latent_in.weight", "cond_in.bias", "double_blocks.1.img_attn.qkv.weight", "double_blocks.0.txt_mlp.2.bias",
               "single_blocks.2.linear2.weight", "single_blocks.0.norm.key_norm.scale", "final_layer.linear.weight"):
@@ -81,12 +68,11 @@ def test_from_pretrained_maps_a_reference_layout_checkpoint(tmp_path, monkeypatc
         assert torch.equal(w["mod.bias"][off:off + n], sd[name + ".bias"]), name
     assert pipe.model.mod_total == 2 * 2 * 6 * H + 3 * 3 * H + 2 * H
     # VAE / geo-decoder / conditioner
-    assert torch.equal(pipe.vae.w["post_kl.weight"], post_kl.weight.detach().half())
+    assert torch.equal(pipe.vae.w["post_kl.weight"], flat["vae.post_kl.weight"])
     assert torch.equal(pipe.vae.w["transformer.resblocks.1.attn.c_qkv.weight"],
-                       tr.state_dict()["resblocks.1.attn.c_qkv.weight"].half())
-    g = geo.state_dict()
-    assert torch.equal(pipe.vae.geo_decoder.w["c_kv.weight"], g["cross_attn_decoder.attn.c_kv.weight"].half())
-    assert torch.equal(pipe.vae.geo_decoder.w["query_proj.weight"][:, :51], g["query_proj.weight"].half())
+                       flat["vae.transformer.resblocks.1.attn.c_qkv.weight"])
+    assert torch.equal(pipe.vae.geo_decoder.w["c_kv.weight"], flat["vae.geo_decoder.cross_attn_decoder.attn.c_kv.weight"])
+    assert torch.equal(pipe.vae.geo_decoder.w["query_proj.weight"][:, :51], flat["vae.geo_decoder.query_proj.weight"])
     assert not pipe.vae.geo_decoder.w["query_proj.weight"][:, 51:].any()      # K padded 51 -> 64 with zeros
     enc = pipe.conditioner.main_image_encoder.model
     assert torch.equal(enc.state_dict()["encoder.layer.1.mlp.weights_in.weight"],

@@ -45,22 +45,17 @@ def test_scheduler_mirror_matches_reference_fixture(golden_dir):
         sch.step(torch.zeros(1), 3, torch.zeros(1))
 
 
-def test_image_processor_against_reference_when_available():
-    import ref_import
-    if not ref_import.available():
-        pytest.skip("/root/reference not present")
+def test_image_processor_against_reference_when_available(golden_dir):
+    """ImageProcessorV2 (preprocessors.py) bit for bit: the reference's image and mask tensors are stored as digests
+    of their bytes (tests/golden/host_helpers.npz)."""
     from PIL import Image
+    from make_golden import ellipse_rgba, sha256
     from r3g.preprocessors import ImageProcessorV2
-    ref = ref_import.hunyuan_preprocessors().ImageProcessorV2(size=512, border_ratio=0.15)
-    rng = np.random.default_rng(0)
-    rgba = np.zeros((300, 420, 4), np.uint8)
-    rgba[..., :3] = rng.integers(0, 256, (300, 420, 3))
-    yy, xx = np.mgrid[0:300, 0:420]
-    rgba[..., 3] = ((((xx - 200) / 120) ** 2 + ((yy - 160) / 90) ** 2) <= 1) * 255
-    img = Image.fromarray(rgba, "RGBA")
-    a, b = ImageProcessorV2(512, 0.15)(img), ref(img)
-    assert torch.equal(a["image"], b["image"]) and torch.equal(a["mask"], b["mask"])
+    z = np.load(os.path.join(golden_dir, "host_helpers.npz"))
+    a = ImageProcessorV2(512, 0.15)(Image.fromarray(ellipse_rgba(), "RGBA"))
     assert a["image"].shape == (1, 3, 512, 512) and a["mask"].shape == (1, 1, 512, 512)
+    assert a["image"].dtype == a["mask"].dtype == torch.float32
+    assert sha256(a["image"]) == z["imgproc_image_sha256"] and sha256(a["mask"]) == z["imgproc_mask_sha256"]
 
 
 def test_stage3_twin_file_contract(tmp_path, monkeypatch):
@@ -97,50 +92,62 @@ def test_bench_reference_arm_contract():
     assert r1.returncode == 0 and r1.stdout.strip() == ""
 
 
-def test_conditioner_mirror_against_reference_when_available():
+def test_bench_dump_outputs_stay_within_64_mb(tmp_path):
+    """`bench.py --dump-outputs`: float32 stays float32 and other dtypes become float64; small arrays are written whole,
+    large ones as the same seeded sample of their rows, in order, on every call; 64 MB in all."""
+    sys.path.insert(0, ROOT)
+    import bench
+
+    def rows(n, dtype):                 # row i holds i three times: a sampled row shows where it came from
+        return np.repeat(np.arange(n, dtype=dtype)[:, None], 3, axis=1)
+    arrays = {"v": rows(3_000_000, np.float32), "f": rows(6_000_000, np.int32), "small": torch.arange(10)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    out = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in arrays}
+    assert sum(os.path.getsize(tmp_path / "a" / f"{k}.npy") for k in arrays) <= 64e6
+    assert out["v"].dtype == np.float32 and out["f"].dtype == np.float64 and out["small"].dtype == np.float64
+    assert np.array_equal(out["small"], np.arange(10))
+    for k in ("v", "f"):
+        a = out[k]
+        assert a.shape[1] == 3 and 0 < len(a) < len(arrays[k])
+        assert (a == a[:, :1]).all() and (np.diff(a[:, 0]) > 0).all()
+    for k in arrays:
+        assert np.array_equal(out[k], np.load(tmp_path / "b" / f"{k}.npy"))
+
+
+def test_conditioner_mirror_against_reference_when_available(golden_dir):
     """Row a2: DinoImageEncoder (conditioner.py:57-131) -- value-range shift, Resize(bilinear, antialias) + CenterCrop +
-    Normalize, HF Dinov2Model, cls token kept; zeros as the unconditional embedding.  Same small random model in both."""
-    ref_path = "/root/reference/Hunyuan3D-2/hy3dgen/shapegen/models/conditioner.py"
-    if not os.path.exists(ref_path):
-        pytest.skip("/root/reference not present")
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("_ref_conditioner", ref_path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    Normalize, HF Dinov2Model, cls token kept; zeros as the unconditional embedding.  Same small seeded model in both;
+    the reference's outputs are in tests/golden/host_helpers.npz."""
     sys.path.insert(0, os.path.join(ROOT, "3d-re-gen_b200"))
     from r3g.conditioner import DinoImageEncoder, SingleImageEncoder
+    from make_golden import seeded_weights
     cfg = dict(hidden_size=32, num_hidden_layers=2, num_attention_heads=2, mlp_ratio=2, patch_size=14, image_size=56,
                use_swiglu_ffn=True, layerscale_value=1.0, qkv_bias=True, hidden_act="gelu", layer_norm_eps=1e-6)
-    torch.manual_seed(0)
-    theirs = ref.DinoImageEncoder(config=cfg, use_cls_token=True, image_size=56)
+    z = np.load(os.path.join(golden_dir, "host_helpers.npz"))
     mine = DinoImageEncoder(config=cfg, use_cls_token=True, image_size=56, device="cpu", dtype=torch.float32)
-    mine.model.load_state_dict(theirs.model.state_dict())
-    for shape in ((1, 3, 70, 90), (2, 3, 100, 64), (1, 3, 56, 56)):
-        img = torch.rand(shape) * 2 - 1
-        a, b = mine(img), theirs(img)
+    mine.model.load_state_dict(seeded_weights({k: v.shape for k, v in mine.model.state_dict().items()}))
+    g = torch.Generator().manual_seed(0)
+    for i, shape in enumerate(((1, 3, 70, 90), (2, 3, 100, 64), (1, 3, 56, 56))):
+        img = torch.rand(shape, generator=g) * 2 - 1
+        a, b = mine(img), torch.from_numpy(z[f"dino_out{i}"])
         assert a.shape == b.shape == (shape[0], 17, 32)
         assert torch.allclose(a, b, atol=1e-5, rtol=1e-5), (a - b).abs().max()
     u = SingleImageEncoder(mine).unconditional_embedding(2)["main"]
-    assert u.shape == (2, 17, 32) and not u.any() and torch.equal(u, theirs.unconditional_embedding(2))
+    assert u.shape == (2, 17, 32) and not u.any() and torch.equal(u, torch.from_numpy(z["dino_uncond"]))
 
 
-def test_near_surface_mask_against_reference_when_available():
-    """extract_near_surface_volume_fn (volume_decoders.py:29-119): the point selection of the FlashVDM levels."""
-    import ref_import
-    if not ref_import.available():
-        pytest.skip("/root/reference not present")
-    import warnings
-    _, _, vd = ref_import.hunyuan_autoencoders()
+def test_near_surface_mask_against_reference_when_available(golden_dir):
+    """extract_near_surface_volume_fn (volume_decoders.py:29-119): the point selection of the FlashVDM levels, against
+    the reference's masks in tests/golden/host_helpers.npz."""
     from r3g.vae import extract_near_surface_volume_fn
+    z = np.load(os.path.join(golden_dir, "host_helpers.npz"))
     torch.manual_seed(0)
     for n in (5, 9):
         x = torch.randn(n, n, n)
         x[torch.rand(n, n, n) < 0.25] = -10000.0
-        for alpha in (0.0, 0.3, -0.2):
-            with warnings.catch_warnings():
-                warnings.simplefilter("ignore")
-                want = vd.extract_near_surface_volume_fn(x, alpha)
-            assert torch.equal(extract_near_surface_volume_fn(x, alpha), want)
+        for j, alpha in enumerate((0.0, 0.3, -0.2)):
+            assert torch.equal(extract_near_surface_volume_fn(x, alpha), torch.from_numpy(z[f"near_surface_{n}_{j}"]))
 
 
 def test_flashvdm_resolution_schedule():

@@ -1,14 +1,11 @@
-"""CPU: pin the oracle restatements (oracle/hy3d_ref.py) against fixtures generated from the REFERENCE's own
-modules (oracle/make_golden.py, run where /root/reference exists) -- and, when the checkout is present,
-against those modules live."""
+"""CPU: pin the oracle restatements (oracle/hy3d_ref.py, oracle/vggt_ref.py) and the VGGT head mirrors against
+fixtures generated from the REFERENCE's own modules (oracle/make_golden.py, run where the reference checkout exists)."""
 import os
 
 import numpy as np
-import pytest
 import torch
 
 import hy3d_ref as R
-import ref_import
 
 
 def load(golden_dir, name):
@@ -73,19 +70,6 @@ def test_unproject_matches_reference_fixture(golden_dir):
     np.testing.assert_allclose(pts, z["points"], rtol=0, atol=1e-12)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="/root/reference not present (GPU box)")
-def test_live_reference_modules_agree_with_fixtures(golden_dir):
-    """Re-run the reference module itself on the fixture inputs: guards the fixtures against drift."""
-    m = ref_import.hunyuan_dit()
-    z, sd = load(golden_dir, "dit_mini.npz")
-    model = m.Hunyuan3DDiT(in_channels=64, context_in_dim=96, hidden_size=128, num_heads=2, depth=2,
-                           depth_single_blocks=2, axes_dim=[64]).eval()
-    model.load_state_dict(sd)
-    with torch.no_grad():
-        y = model(torch.from_numpy(z["x"]), torch.from_numpy(z["t"]), {"main": torch.from_numpy(z["cond"])})
-    np.testing.assert_allclose(y.numpy(), z["y"], rtol=0, atol=1e-6)
-
-
 def test_vggt_restatement_matches_reference_fixture(golden_dir):
     import vggt_ref as V
     z = np.load(os.path.join(golden_dir, "vggt_mini.npz"))
@@ -99,40 +83,27 @@ def test_vggt_restatement_matches_reference_fixture(golden_dir):
         np.testing.assert_allclose(y.numpy(), z[f"vit_y_{tag}"], rtol=0, atol=3e-5)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="/root/reference not present (GPU box)")
-def test_vggt_heads_mirror_matches_reference_modules_live():
-    """The torch-operator mirrors of CameraHead / DPTHead / pose utilities against the reference modules (CPU, fp32)."""
+def test_vggt_heads_mirror_matches_reference_modules_live(golden_dir):
+    """The torch-operator mirrors of CameraHead / DPTHead / pose utilities against the reference modules' outputs
+    (CPU, fp32) on seeded weights of the reference heads' layout (tests/golden/vggt_heads_mini.npz)."""
     import sys
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "3d-re-gen_b200"))
-    ref_import.vggt_package()
-    from vggt.heads.camera_head import CameraHead as RefCam
-    from vggt.heads.dpt_head import DPTHead as RefDPT
-    from vggt.utils.pose_enc import pose_encoding_to_extri_intri as ref_pose
+    from make_golden import seeded_weights, stored_layout
     from r3g import vggt_heads as M
-    torch.manual_seed(0)
+    z = np.load(os.path.join(golden_dir, "vggt_heads_mini.npz"))
+    sd = seeded_weights(stored_layout(z))
     C, S, H, W = 128, 2, 56, 70
     ph, pw = H // 14, W // 14
+    torch.manual_seed(0)
     toks = [torch.randn(1, S, 5 + ph * pw, C) for _ in range(4)]
-    cam = RefCam(dim_in=C, trunk_depth=2, num_heads=2).eval()
-    with torch.no_grad():
-        for n, p in cam.named_parameters():
-            if "gamma" in n or n == "empty_pose_tokens":
-                p.copy_(0.3 * torch.randn_like(p))
-        ref = cam(toks)
-    mine = M.CameraHead({"camera_head." + k: v for k, v in cam.state_dict().items()}, trunk_depth=2, num_heads=2,
-                        device="cpu")(toks)
-    for a, b in zip(mine, ref):
-        np.testing.assert_allclose(a.numpy(), b.numpy(), rtol=0, atol=2e-5)
-    e1, k1 = M.pose_encoding_to_extri_intri(mine[-1], (H, W))
-    e2, k2 = ref_pose(ref[-1], (H, W))
-    np.testing.assert_allclose(e1.numpy(), e2.numpy(), atol=1e-5)
-    np.testing.assert_allclose(k1.numpy(), k2.numpy(), rtol=1e-5)
-    dpt = RefDPT(dim_in=C, output_dim=2, activation="exp", conf_activation="expp1", features=32,
-                 out_channels=[16, 32, 64, 64], intermediate_layer_idx=[0, 1, 2, 3]).eval()
     imgs = torch.rand(1, S, 3, H, W)
-    with torch.no_grad():
-        rd, rc = dpt(toks, images=imgs, patch_start_idx=5)
-    md, mc = M.DPTHead({"depth_head." + k: v for k, v in dpt.state_dict().items()}, intermediate_layer_idx=(0, 1, 2, 3),
-                       device="cpu")(toks, imgs, 5)
-    np.testing.assert_allclose(md.numpy(), rd.numpy(), rtol=1e-4, atol=1e-5)
-    np.testing.assert_allclose(mc.numpy(), rc.numpy(), rtol=1e-4, atol=1e-5)
+    mine = M.CameraHead(sd, trunk_depth=2, num_heads=2, device="cpu")(toks)
+    assert len(mine) == 4
+    for i, a in enumerate(mine):
+        np.testing.assert_allclose(a.numpy(), z[f"pose{i}"], rtol=0, atol=2e-5)
+    e1, k1 = M.pose_encoding_to_extri_intri(mine[-1], (H, W))
+    np.testing.assert_allclose(e1.numpy(), z["extrinsic"], atol=1e-5)
+    np.testing.assert_allclose(k1.numpy(), z["intrinsic"], rtol=1e-5)
+    md, mc = M.DPTHead(sd, intermediate_layer_idx=(0, 1, 2, 3), device="cpu")(toks, imgs, 5)
+    np.testing.assert_allclose(md.numpy(), z["depth"], rtol=1e-4, atol=1e-5)
+    np.testing.assert_allclose(mc.numpy(), z["conf"], rtol=1e-4, atol=1e-5)

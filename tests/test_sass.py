@@ -15,18 +15,20 @@ LIB = os.path.join(ROOT, "3d-re-gen_b200", "r3g", "libr3g.so")
 
 @pytest.fixture(scope="module")
 def sass():
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
+    # the CUDA toolkit's own location when it is not on PATH, as the build does for nvcc
+    cuobjdump = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
+    if not os.path.exists(cuobjdump):
+        pytest.skip("cuobjdump not found")
     import sys
     sys.path.insert(0, ROOT)
     import __graft_entry__ as ge
     ge.build()
-    txt = subprocess.run(["cuobjdump", "-sass", LIB], capture_output=True, text=True, check=True).stdout
+    txt = subprocess.run([cuobjdump, "-sass", LIB], capture_output=True, text=True, check=True).stdout
     funcs = {}
     for blk in re.split(r"\n\s*Function : ", txt)[1:]:
         name, _, body = blk.partition("\n")
         funcs[name.strip()] = body
-    res = subprocess.run(["cuobjdump", "-res-usage", LIB], capture_output=True, text=True, check=True).stdout
+    res = subprocess.run([cuobjdump, "-res-usage", LIB], capture_output=True, text=True, check=True).stdout
     usage = {m.group(1): (int(m.group(2)), int(m.group(3)))
              for m in re.finditer(r"Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+)", res)}
     return funcs, usage
